@@ -1,8 +1,14 @@
 #!/usr/bin/env python
 """bench.py - sequences/sec of one biGRU train step on N B200s (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32] [--dump-outputs DIR]
   N>1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N
+
+--dump-outputs DIR writes what the last timed step of the headline returned, DIR/loss.npy and DIR/logits.npy (float32), so that
+two builds run with the same arguments (same seeded inputs and initial parameters) can be compared output for output.  Compare
+with a tolerance: the split-K reductions do not sum in a fixed order and Adam turns last-bit gradient differences into
+lr-sized steps, so two runs of one build differ (NVIDIA B200, 1000 W limit, --steps 20 --warmup 5, two pairs of runs: loss
+by up to 1.3e-4 relative, logits by up to 8e-3 of their largest magnitude).
 
 A "step" is the body of the reference training loop (biGRU_model.py:198-210): zero_grad -> forward ->
 CrossEntropy loss -> backward -> [gradient all-reduce] -> clip_grad_norm_(50) -> Adam, on the workload
@@ -26,6 +32,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 METRIC = "sequences/sec (train step) biGRU h=256 seq=128 feat=64"
 WORK = dict(per_gpu_batch=512, seq_len=128, n_features=64, hidden=256, layers=2, classes=3)
@@ -197,7 +204,13 @@ def main():
     ap.add_argument("--no-variants", action="store_true", help="skip the secondary precision (bf16) measurement")
     ap.add_argument("--config", default="c1", choices=["c1", "c4"],
                     help="c1: BASELINE.json configs[1] (the headline metric); c4: configs[4] long sequence (B256 T1024 F128 H512)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and logits of the headline's last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     global WORK, METRIC
     if args.config == "c4":
         WORK, METRIC = WORK_C4, METRIC_C4
@@ -280,15 +293,16 @@ def main():
             ms = max_over_ranks(ms, dev)
         return ms, launches
 
-    def measure(prec, steps, warmup, with_e2e=True, with_roofline=True, clocks=False):
+    def measure(prec, steps, warmup, with_e2e=True, with_roofline=True, clocks=False, keep_outputs=False):
         """value (device-resident inputs), e2e (pinned host inputs, H2D + loss D2H inside the timed region) and the live
         per-kernel-class roofline of one precision."""
         model = make_model(prec)
         out = {"precision": prec, "workload": (CONFIG_OF_C4 if args.config == "c4" else CONFIG_OF).get(prec)}
+        last = [None]
 
         def step_resident(i):
             x, t = resident[i % NBUF]
-            model.train_step(x, t)
+            last[0] = model.train_step(x, t)
 
         sampler = ClockSampler(local)
         if clocks and rank == 0:
@@ -297,6 +311,8 @@ def main():
         ms, launches = timed(step_resident, steps, warmup)
         if clocks:
             out["clocks"] = sampler.stop() if rank == 0 else None
+        if keep_outputs:
+            out["_outputs"] = {k: v.float().cpu().numpy() for k, v in zip(("loss", "logits"), last[0])}
         ms_step = ms / steps
         out.update(value=B * world / (ms_step * 1e-3), ms_per_step=ms_step, gpu_launches=int(launches))
         if world > 1:
@@ -428,8 +444,9 @@ def main():
         out["_model"] = model
         return out
 
-    head = measure(precision, args.steps, args.warmup, clocks=True)
+    head = measure(precision, args.steps, args.warmup, clocks=True, keep_outputs=bool(args.dump_outputs))
     model = head.pop("_model")
+    outputs = head.pop("_outputs", None)
 
     # ---- end to end THROUGH THE LOADER (SURVEY 8(f) N1): a host chunk -> device -> zero-copy windows ----------------
     e2e_windows = None
@@ -549,9 +566,19 @@ def main():
                 "config": workload_config(world, precision), "clocks": head.get("clocks"), "e2e": head.get("e2e"),
                 "gpu_launches": head["gpu_launches"], "roofline": head.get("roofline"), "cpu_baseline": cpu,
                 "e2e_windows": e2e_windows, "variants": variants, "parity": parity, "cudnn_comparator": cudnn, "comm": head.get("comm")}
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         _emit(line)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(directory, arrays):
+    """One DIR/<name>.npy per array."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def _emit(obj):

@@ -1,6 +1,6 @@
 """Pins the SQL window-function features (SURVEY.md 8(f) N4) to the REFERENCE'S OWN SQL.
 
-The reference builds its feature views as SQL strings inside /root/reference/create_database.py (:76-190) and executes
+The reference builds its feature views as SQL strings inside create_database.py (:76-190) and executes
 them on a MariaDB server at import time.  No MariaDB here - but the statements are plain window-function SQL, so this
 script imports the UNMODIFIED module with
   * a stub `mysql.connector` whose cursor forwards every statement to an in-memory sqlite3 database (a dialect shim only:
@@ -11,7 +11,7 @@ script imports the UNMODIFIED module with
 fills `stock_data_joined` with a seed-fixed synthetic market table (values exactly representable in the FLOAT(6,2) / INT
 columns the reference declares) and selects every view plus the `target` view.  Output: tests/golden/features.npz.
 
-Run in the build container:  python tests/golden/make_features_golden.py
+  python tests/golden/make_features_golden.py REFERENCE_DIR      (a checkout of the original project)
 """
 import math
 import os
@@ -22,7 +22,9 @@ import types
 
 import numpy as np
 
-REF = "/root/reference"
+if len(sys.argv) != 2:
+    sys.exit(__doc__)
+REF = os.path.abspath(sys.argv[1])
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "features.npz")
 
 

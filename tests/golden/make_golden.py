@@ -1,11 +1,13 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference from /root/reference.
+"""Generates tests/golden/*.npz by running the UNMODIFIED reference (a checkout of the original project).
 
-Run in the build container only (python tests/golden/make_golden.py); /root/reference does not
-exist on the GPU box, so the fixtures are committed.  Nothing here is imported by the product.
+  python tests/golden/make_golden.py REFERENCE_DIR
+
+The fixtures are committed, so the tests never need the reference.  Nothing here is imported by the product.
 
   kat.npz          shipped model_params.pt (H=8,F=108,C=4,L=1) + two fixed inputs -> logits
   model_<case>.npz seed-fixed synthetic cases through reference BiGRU: inputs, state_dict,
                    logits, loss, every gradient, (dx, dh0), params after clip+Adam
+                   (model_c0 in the compact form that tests/golden_cases.py reads)
   loader.npz       reference MySQLChunkLoader / MySQLBatchLoader / TrainValTestSplit driven by
                    tests/fake_db.FakeCursor: chunk ranges, norm params, delivered batches
 """
@@ -19,9 +21,13 @@ import torch
 import torch.nn as nn
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+if len(sys.argv) != 2:
+    sys.exit(__doc__)
+REF = os.path.abspath(sys.argv[1])
 sys.path.insert(0, os.path.dirname(HERE))
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, REF)
 import fake_db  # noqa: E402
+import golden_cases  # noqa: E402
 
 fake_db.install_reference_stubs(bid_levels=2, ask_levels=2)
 from biGRU_model import BiGRU  # noqa: E402  (reference, unmodified)
@@ -35,7 +41,7 @@ def sd_np(sd, prefix):
 
 
 def gen_kat():
-    sd = torch.load("/root/reference/model_params.pt", map_location="cpu")
+    sd = torch.load(os.path.join(REF, "model_params.pt"), map_location="cpu")
     m = BiGRU(8, 108, 4, 1, 50, 0.2, False, True)
     m.load_state_dict(sd)
     m.eval()
@@ -47,7 +53,7 @@ def gen_kat():
         out = {"x1": x1.numpy(), "y1": m(x1).numpy(), "x2": x2.numpy(), "y2": m(x2).numpy(),
                "x3": x3.numpy(), "y3": m(x3).numpy()}
     out.update(sd_np(sd, "p:"))
-    with open("/root/reference/norm_params", "rb") as f:
+    with open(os.path.join(REF, "norm_params"), "rb") as f:
         npar = pickle.load(f)
     out["norm_min"] = np.array([float(v["MIN"]) for v in npar.values()], np.float32)
     out["norm_max"] = np.array([float(v["MAX"]) for v in npar.values()], np.float32)
@@ -55,7 +61,22 @@ def gen_kat():
     print("kat", out["y1"], out["y2"])
 
 
-def gen_model(name, B, T, F, H, L, C, bidir, loss, with_h0=False, seed=1234):
+def compact(out, seed):
+    """Keeps model_c0 under 1 MB (its float32 arrays do not compress): the inputs are left out - tests/golden_cases.py
+    rebuilds them from the two seeds and checks them against inputs_sha256 - and the parameters after the step are stored
+    as their difference from the initial ones (an exact round trip, asserted here)."""
+    names = [k[2:] for k in out if k.startswith("p:")]
+    out["input_seeds"] = np.array([0, seed], np.int64)
+    out["inputs_sha256"] = np.array(golden_cases.inputs_sha256(out["x"], [out["p:" + k] for k in names]))
+    for k in names:
+        p, q = out.pop("p:" + k), out.pop("q:" + k)
+        dq = (q.astype(np.float64) - p).astype(np.float32)
+        assert np.array_equal(p + dq, q), k
+        out["dq:" + k] = dq
+    del out["x"]
+
+
+def gen_model(name, B, T, F, H, L, C, bidir, loss, with_h0=False, seed=1234, rebuilt_inputs=False):
     torch.manual_seed(0)
     m = BiGRU(H, F, C, L, 50, 0.0, False, bidir)
     g = torch.Generator().manual_seed(seed)
@@ -98,6 +119,8 @@ def gen_model(name, B, T, F, H, L, C, bidir, loss, with_h0=False, seed=1234):
     out.update(sd_np(m.state_dict(), "q:"))          # params after one clip+Adam step
     out["meta"] = np.array([B, T, F, H, L, C, int(bidir)], np.int64)
     out["loss_kind"] = np.array(loss)
+    if rebuilt_inputs:
+        compact(out, seed)
     np.savez_compressed(os.path.join(HERE, f"model_{name}.npz"), **out)
     print(name, "loss", lv.item(), "norm", float(norm))
 
@@ -142,7 +165,7 @@ def gen_loader():
 
 if __name__ == "__main__":
     gen_kat()
-    gen_model("c0", 32, 64, 32, 128, 1, 3, True, "ce")                 # BASELINE config 0
+    gen_model("c0", 32, 64, 32, 128, 1, 3, True, "ce", rebuilt_inputs=True)    # BASELINE config 0
     gen_model("small_l2", 4, 7, 5, 8, 2, 3, True, "ce")
     gen_model("small_uni_bce", 3, 6, 4, 8, 2, 4, False, "bce", with_h0=True)
     gen_model("small_bi_h0_mlsm", 5, 9, 12, 16, 2, 4, True, "mlsm", with_h0=True)

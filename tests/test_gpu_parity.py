@@ -9,6 +9,7 @@ import torch
 import torch.nn as nn
 
 import fake_db
+import golden_cases
 import oracle_c
 from oracle import bigru_oracle as bo
 from oracle import loader_oracle as lo
@@ -68,7 +69,7 @@ def rel_l2(a, b):
 
 
 def params_of(z, prefix="p:"):
-    return {k[len(prefix):]: z[k] for k in z.files if k.startswith(prefix)}
+    return {k[len(prefix):]: z[k] for k in z if k.startswith(prefix)}
 
 
 def make_model(d, sd_np, precision, dropout=0.0, spatial=False):
@@ -111,17 +112,17 @@ def test_known_answer_vectors(golden_dir):
 @pytest.mark.parametrize("name", ["c0", "small_l2", "small_uni_bce", "small_bi_h0_mlsm", "ragged"])
 def test_golden_forward_backward_autograd(golden_dir, name):
     """Logits, loss, every parameter gradient, dx and dh0 against the reference's own autograd."""
-    z = np.load(os.path.join(golden_dir, f"model_{name}.npz"))
+    z = golden_cases.load(golden_dir, name)
     B, T, F, H, L, C, bidir = [int(v) for v in z["meta"]]
     d = dict(B=B, T=T, F=F, H=H, L=L, C=C, bidir=bool(bidir))
     for precision in precisions():
-        if not supported(precision, B, F, H, "h0" in z.files):
+        if not supported(precision, B, F, H, "h0" in z):
             continue
         tol = TOL[precision]
         m = make_model(d, params_of(z), precision)
         m.train()
         x = torch.from_numpy(z["x"]).cuda().requires_grad_(True)
-        h0 = torch.from_numpy(z["h0"]).cuda().requires_grad_(True) if "h0" in z.files else None
+        h0 = torch.from_numpy(z["h0"]).cuda().requires_grad_(True) if "h0" in z else None
         loss_fn, tgt = loss_from(z)
         loss_fn = loss_fn.cuda()
         pred = m(x, h0)
@@ -144,11 +145,11 @@ def test_golden_forward_backward_autograd(golden_dir, name):
 def test_golden_fused_train_step(golden_dir, name):
     """zero_grad -> forward -> loss -> backward -> clip_grad_norm_ -> Adam (biGRU_model.py:198-210):
     parameters after one fused step against the reference's."""
-    z = np.load(os.path.join(golden_dir, f"model_{name}.npz"))
+    z = golden_cases.load(golden_dir, name)
     B, T, F, H, L, C, bidir = [int(v) for v in z["meta"]]
     d = dict(B=B, T=T, F=F, H=H, L=L, C=C, bidir=bool(bidir))
     for precision in precisions():
-        if not supported(precision, B, F, H, "h0" in z.files):
+        if not supported(precision, B, F, H, "h0" in z):
             continue
         tol = TOL[precision]
         m = make_model(d, params_of(z), precision)
@@ -156,7 +157,7 @@ def test_golden_fused_train_step(golden_dir, name):
         m.add_loss_fn(loss_fn)
         m.add_optimizer(torch.optim.Adam(m.parameters(), lr=1e-3))
         m.train()
-        h0 = torch.from_numpy(z["h0"]).cuda() if "h0" in z.files else None
+        h0 = torch.from_numpy(z["h0"]).cuda() if "h0" in z else None
         loss, logits = m.train_step(torch.from_numpy(z["x"]).cuda(), tgt.cuda(), h0)
         assert abs(float(loss) - float(z["loss"])) < 10 * tol["logits"] * max(1.0, abs(float(z["loss"])))
         assert rel(logits.cpu().numpy(), z["logits"]) < tol["logits"]
@@ -164,10 +165,10 @@ def test_golden_fused_train_step(golden_dir, name):
         assert abs(gn - float(z["grad_norm"])) < tol["grads"] * float(z["grad_norm"])
         upd_got, upd_ref = [], []
         for k, v in m.state_dict().items():
-            if "q:" + k not in z.files:
+            if "q:" + k not in z:
                 continue
             assert np.abs(v.cpu().numpy() - z["q:" + k]).max() < tol["step"], (precision, k)
-            if "q:" + k not in z.files:
+            if "q:" + k not in z:
                 continue                                  # buffers of the attached loss module
             upd_got.append((v.cpu().numpy() - z["p:" + k]).ravel())
             upd_ref.append((z["q:" + k] - z["p:" + k]).ravel())

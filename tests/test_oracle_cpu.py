@@ -8,6 +8,7 @@ import pytest
 import torch
 import torch.nn as nn
 
+import golden_cases
 import oracle_c
 from oracle import bigru_oracle as bo
 from oracle import loader_oracle as lo
@@ -17,13 +18,13 @@ CASES = ["c0", "small_l2", "small_uni_bce", "small_bi_h0_mlsm", "ragged"]
 
 
 def load(golden_dir, name):
-    z = np.load(os.path.join(golden_dir, f"model_{name}.npz"))
+    z = golden_cases.load(golden_dir, name)
     B, T, F, H, L, C, bidir = [int(v) for v in z["meta"]]
     return z, dict(B=B, T=T, F=F, H=H, L=L, C=C, D=2 if bidir else 1, bidir=bool(bidir))
 
 
 def params_of(z, prefix="p:"):
-    return {k[len(prefix):]: z[k] for k in z.files if k.startswith(prefix)}
+    return {k[len(prefix):]: z[k] for k in z if k.startswith(prefix)}
 
 
 def test_kat_torch_oracle(golden_dir):
@@ -66,7 +67,7 @@ def test_c_oracle_forward_backward(golden_dir, name):
     z, d = load(golden_dir, name)
     P = params_of(z)
     flat = oracle_c.flatten_params(P, d["L"], d["D"])
-    h0 = z["h0"] if "h0" in z.files else None
+    h0 = z["h0"] if "h0" in z else None
     logits, hn, stash = oracle_c.forward(flat, z["x"], d["H"], d["L"], d["C"], d["D"], h0, keep=True)
     scale = np.abs(z["logits"]).max()
     assert np.abs(logits - z["logits"]).max() / scale < 2e-6
@@ -90,7 +91,7 @@ def test_c_oracle_forward_backward(golden_dir, name):
 def test_numpy_equations(golden_dir, name):
     z, d = load(golden_dir, name)
     P = params_of(z)
-    h0 = z["h0"] if "h0" in z.files else None
+    h0 = z["h0"] if "h0" in z else None
     logits, cache = bo.gru_forward_np(P, z["x"], d["H"], d["L"], d["bidir"], h0, keep=True)
     np.testing.assert_allclose(logits, z["logits"], atol=3e-6, rtol=0)
     _, dlog = _loss_and_dlogits(z, z["logits"])
