@@ -207,6 +207,10 @@ class BiGRU(nn.Module):
                 run zero-padded, any feature count),
       "bf16"    single bf16 operands on tcgen05, fp32 accumulation and state (fastest, ~3e-3 on logits); H in {128, 256, 512},
       "auto"    "bf16x3" for hidden sizes up to 256 (smaller models run zero-padded to 128 / 256 hidden units), "fp32" beyond.
+    Every precision takes an initial hidden state (``forward(input_seq, hidden)``, ``train_step(x, target, hidden)``) and returns
+    its gradient through autograd; on the tensor-core paths W_hh·hidden is formed in fp32 and hidden enters the first step's gate
+    math and dW_hh in fp32 (the smaller models' zero padding extends to it).
+    A train step with ``hidden`` runs as plain launches (CUDA-graph replay is for steps without it).
     Default: $BIGRU_B200_PRECISION or "auto" (the reference tolerance at tensor-core speed wherever the kernels apply).
     """
 

@@ -3,8 +3,10 @@
 //   recurrences forward / backward              : tc_scan.cuh  (persistent cluster kernels, W_hh resident in tensor memory)
 //   head, loss glue, optimiser                  : the fp32 kernels of kernels_f32.cuh
 // All activations inside this path are TIME-MAJOR (row r = t*B + b) so that one step of one batch tile is a
-// contiguous block of rows.  Supported: H in {128, 256}, B % 16 == 0, F % 8 == 0, no initial hidden state;
-// anything else fails with BIGRU_ERR_UNSUPPORTED (the fp32 path covers the general case).
+// contiguous block of rows.  Supported: H in {128, 256} with B % 16 == 0 and H = 512 with B % 32 == 0, any F (K extent padded
+// to 8), with or without an initial hidden state; anything else fails with BIGRU_ERR_UNSUPPORTED (the fp32 path covers the
+// general case).  An initial state enters as in path_x3.cuh: W_hh h0 is formed once per layer in fp32 (FFMA GEMM) and the scans
+// read it at step 0, which has no recurrent MMA; the backward scans run one more product for d(h0).
 #pragma once
 #include "common.cuh"
 #include "kernels_f32.cuh"
@@ -31,7 +33,7 @@ struct Bf16Layout {            // byte offsets, 1024-aligned
     size_t Yrow[16], YB[16], G[16], Xrow[16];                    // stash: activations
     size_t Wih[16], WihT[16], Wimg[16], WTimg[16], bfold[16], bhn[16];   // stash: packed weights
     size_t cat, arg, dbg, stash_total;
-    size_t gi, dghn, dYa, dYb, dcat, dhinit, scratch_total;
+    size_t gi, dghn, dYa, dYb, dcat, dhinit, gh0, scratch_total;
 };
 static inline size_t al(size_t x) { return (x + 1023) & ~(size_t)1023; }
 // Layer-0 operands (X rows and W_ih rows) are stored with their K extent (n_features) padded to a multiple of 8 with zeros: a
@@ -66,6 +68,7 @@ static Bf16Layout bf16_layout(const bigru_plan& p) {
     L.dYb = o; o = al(o + R * wide * 4);
     L.dcat = o; o = al(o + (size_t)p.B * 3 * H * 4);
     L.dhinit = o; o = al(o + D * (size_t)p.B * H * 4);
+    L.gh0 = o; o = al(o + (size_t)p.B * D * 3 * H * 4);          // W_hh h0 of the layer being scanned (initial state given)
     L.scratch_total = o;
     return L;
 }
@@ -394,6 +397,41 @@ __global__ void head_bwd_w_kernel(const float* __restrict__ dlogits, const float
     if (k == 0) atomicAdd(dlin_b + cc, accb);
 }
 
+// dW_hh[d] += dgh_first^T h0[d]: the first forward step's h_prev is the caller's initial state, which the time-shifted
+// Y operand of the dW_hh GEMM does not contain (it reads zeros there).  dgh = [da_r | da_z] (dgi rows) and da_n * r (dghn rows),
+// bf16; the bf16x3 path passes the residual parts as well (dgh = hi + lo), this path passes lo = nullptr.
+// Thread = gate row q x DWHH_H0_COLS consecutive columns (one dgh load feeds that many FMAs); grid ((3H+127)/128, H/DWHH_H0_COLS, D).
+constexpr int DWHH_H0_COLS = 8;                               // H % 8 == 0 on the tensor-core paths
+__global__ void dwhh_h0_kernel(const bf16_t* __restrict__ dgi_hi, const bf16_t* __restrict__ dgi_lo, const bf16_t* __restrict__ dghn_hi,
+                               const bf16_t* __restrict__ dghn_lo, const float* __restrict__ h0, float* __restrict__ dwhh, int64_t dir_stride,
+                               int B, int T, int H, int D) {
+    const int d = blockIdx.z;
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;      // gate row of W_hh (0..3H)
+    const int k0 = blockIdx.y * DWHH_H0_COLS;                 // first column of W_hh
+    if (q >= 3 * H) return;
+    const int64_t t_first = d == 0 ? 0 : T - 1;
+    float acc[DWHH_H0_COLS];
+#pragma unroll
+    for (int j = 0; j < DWHH_H0_COLS; ++j) acc[j] = 0.f;
+    for (int b = 0; b < B; ++b) {
+        const int64_t row = t_first * B + b;
+        float g;
+        if (q < 2 * H) {
+            const int64_t i = row * D * 3 * H + d * 3 * H + q;
+            g = dgi_lo ? __bfloat162float(dgi_hi[i]) + __bfloat162float(dgi_lo[i]) : __bfloat162float(dgi_hi[i]);
+        } else {
+            const int64_t i = row * D * H + d * H + q - 2 * H;
+            g = dghn_lo ? __bfloat162float(dghn_hi[i]) + __bfloat162float(dghn_lo[i]) : __bfloat162float(dghn_hi[i]);
+        }
+        const float* hb = h0 + ((int64_t)d * B + b) * H + k0;
+#pragma unroll
+        for (int j = 0; j < DWHH_H0_COLS; ++j) acc[j] = fmaf(g, hb[j], acc[j]);
+    }
+    float* w = dwhh + (int64_t)d * dir_stride + (int64_t)q * H + k0;
+#pragma unroll
+    for (int j = 0; j < DWHH_H0_COLS; ++j) w[j] += acc[j];
+}
+
 // dX^T of layer 0 (fp32 [F][R]) back to the caller's [B][T][F] (+ input-dropout mask); 32x32 smem transpose
 __global__ void dx_to_batch_major_kernel(const float* __restrict__ dXT, float* __restrict__ dx, int B, int T, int F,
                                          float pdrop, int spatial, uint64_t seed) {
@@ -457,7 +495,6 @@ static inline unsigned nblk2(int64_t n, int bs) { return (unsigned)cdiv64(n, bs)
 static int forward_bf16(const bigru_plan& p, const float* params, const float* x, const float* h0, float drop,
                         int spatial, int training, uint64_t seed, void* stash_v, void* scratch_v, float* logits,
                         float* hn, cudaStream_t st, WindowSrc win = WindowSrc{nullptr, nullptr, nullptr, 0}) {
-    if (h0) { bigru_set_error("BIGRU_PREC_BF16: an initial hidden state is not supported; use BIGRU_PREC_FP32"); return BIGRU_ERR_UNSUPPORTED; }
     const Bf16Layout L = bf16_layout(p);
     const bool wide = bf16_wide(p);
     uint8_t* S = (uint8_t*)stash_v;
@@ -528,7 +565,14 @@ static int forward_bf16(const bigru_plan& p, const float* params, const float* x
             g.b_win = wnd ? B : 0;
             TRY(tc_gemm(S + L.Wih[l], D * 3 * H, Ip, Xrow, wnd ? (int64_t)B + T - 1 : R, Ip, g, st));
         }
-        // 4. recurrence
+        // 4. recurrence.  With an initial state its recurrent product W_hh h0 is formed here in fp32 (tiny: B x 3H x H per
+        //    direction, no bias) and read by the scan at step 0, which issues no recurrent MMA.
+        const float* h0l = h0 ? h0 + (int64_t)l * D * B * H : nullptr;
+        if (h0l) {
+            GemmArgs r = gemm_args(h0l, params + p.off_whh(l, 0), (float*)(W + L.gh0), B, 3 * H, H, H, 1, H, 1, 3 * H);
+            r.batch = D; r.zA = (int64_t)B * H; r.zB = p.ld_block(l); r.zC = (int64_t)B * 3 * H;
+            TRY(sgemm_launch(r, st));
+        }
         if (wide) {
             using WG = tcw::Geo<512>;
             tcw::FwdParams f{};
@@ -537,6 +581,7 @@ static int forward_bf16(const bigru_plan& p, const float* params, const float* x
             f.giW = (const bf16_t*)(W + L.gi); f.b_hn = (const float*)(S + L.bhn[l]);
             f.Yrow = (bf16_t*)(S + L.Yrow[l]); f.GW = (bf16_t*)(S + L.G[l]); f.YBW = (bf16_t*)(S + L.YB[l]);
             f.hn_out = hn ? hn + (int64_t)l * D * B * H : nullptr; f.dbg = dbg;
+            f.h0 = h0l; f.gh0 = h0l ? (const float*)(W + L.gh0) : nullptr;
             ProfScope ps(KC_TC_SCAN_FWD, 2.0 * 3 * H * H * (double)R * D, 0.0, st);
             CUDA_TRY(tcw::launch_fwd(f, st));
             continue;
@@ -546,6 +591,7 @@ static int forward_bf16(const bigru_plan& p, const float* params, const float* x
         f.Wimg = (const bf16_t*)(S + L.Wimg[l]); f.giB = (const bf16_t*)(W + L.gi); f.b_hn = (const float*)(S + L.bhn[l]);
         f.Yrow = (bf16_t*)(S + L.Yrow[l]); f.G = (bf16_t*)(S + L.G[l]); f.YB = (bf16_t*)(S + L.YB[l]);
         f.hn_out = hn ? hn + (int64_t)l * D * B * H : nullptr; f.dbg = dbg;
+        f.h0 = h0l; f.gh0 = h0l ? (const float*)(W + L.gh0) : nullptr;
         f.fuse_x = fuse_x ? 1 : 0; f.x_win = (direct && l == 0) ? 1 : 0; f.Xrow = Xrow; f.Wih = (const bf16_t*)(S + L.Wih[l]); f.bfold = (const float*)(S + L.bfold[l]);
         {
             ProfScope ps(KC_TC_SCAN_FWD, 2.0 * 3 * H * H * (double)R * D, 0.0, st);
@@ -573,7 +619,6 @@ static int backward_bf16(const bigru_plan& p, const float* params, const float* 
     // vector and forms the head's gradients; a later call for the lower layers continues from the dY the upper call left in scratch.
     if (l_from < 0) l_from = p.L - 1;
     const bool from_top = l_from == p.L - 1;
-    if (h0 || dh0) { bigru_set_error("BIGRU_PREC_BF16: initial hidden state / its gradient are not supported"); return BIGRU_ERR_UNSUPPORTED; }
     const Bf16Layout L = bf16_layout(p);
     const bool wide = bf16_wide(p);
     const uint8_t* S = (const uint8_t*)stash_v;
@@ -594,12 +639,14 @@ static int backward_bf16(const bigru_plan& p, const float* params, const float* 
     if ((p.L - 1 - l_from) & 1) { float* t_ = dY; dY = dYnext; dYnext = t_; }      // the buffers alternate per layer
     for (int l = l_from; l >= l_to; --l) {
         const int I = (int)p.in_size(l);
+        const float* h0l = h0 ? h0 + (int64_t)l * D * B * H : nullptr;
+        float* dh0l = dh0 ? dh0 + (int64_t)l * D * B * H : nullptr;
         // 1. BPTT scan
         if (wide) {
             tcw::BwdParams b{};
             b.B = B; b.T = T; b.H = H; b.D = D;
             b.WTimg = (const bf16_t*)(S + L.WTimg[l]); b.GW = (const bf16_t*)(S + L.G[l]); b.YBW = (const bf16_t*)(S + L.YB[l]);
-            b.dYBW = dY;
+            b.dYBW = dY; b.h0 = h0l; b.dh0 = dh0l;
             if (l == p.L - 1) { b.dlogits = dlogits; b.lin_w = params + p.off_linw(); b.arg = (const int*)(S + L.arg); b.C = C; }
             b.dgi_row = (bf16_t*)(W + L.gi); b.dghn_row = (bf16_t*)(W + L.dghn);
             b.db_ih = grads + p.off_bih(l, 0); b.db_hh = grads + p.off_bhh(l, 0); b.dir_stride = p.ld_block(l); b.dbg = dbg;
@@ -609,7 +656,7 @@ static int backward_bf16(const bigru_plan& p, const float* params, const float* 
             tcs::BwdParams b{};
             b.B = B; b.T = T; b.H = H; b.D = D;
             b.WTimg = (const bf16_t*)(S + L.WTimg[l]); b.G = (const bf16_t*)(S + L.G[l]); b.YB = (const bf16_t*)(S + L.YB[l]);
-            b.dYB = dY;
+            b.dYB = dY; b.h0 = h0l; b.dh0 = dh0l;
             if (l == p.L - 1) { b.dlogits = dlogits; b.lin_w = params + p.off_linw(); b.arg = (const int*)(S + L.arg); b.C = C; }
             b.dgi_row = (bf16_t*)(W + L.gi); b.dghn_row = (bf16_t*)(W + L.dghn);
             b.db_ih = grads + p.off_bih(l, 0); b.db_hh = grads + p.off_bhh(l, 0); b.dir_stride = p.ld_block(l); b.dbg = dbg;
@@ -634,8 +681,8 @@ static int backward_bf16(const bigru_plan& p, const float* params, const float* 
             TRY(tc_gemm(W + L.gi, (int64_t)D * 3 * H, (int64_t)D * 3 * H, Xin, I, pad8(I), g, st, KC_TC_GEMM_DWIH));   // I columns, padded row pitch
         }
         // 3. dW_hh[d] = dgh[d]^T H_prev  with H_prev(t) = Y(t-1) (dir 0) / Y(t+1) (dir 1): a shift of -+B ROWS of the
-        //    time-major output; rows outside [0, R) read as zero through TMA (h_prev = 0 at the first step).
-        //    dgh = [da_r | da_z] (columns of dgi_row) and da_n*r (dghn_row): two launches.
+        //    time-major output; rows outside [0, R) read as zero through TMA (h_prev = 0 at the first step; an initial state's
+        //    term is added by dwhh_h0_kernel below).  dgh = [da_r | da_z] (columns of dgi_row) and da_n*r (dghn_row): two launches.
         for (int part = 0; part < 2; ++part) {
             tcg::Params g{};
             g.M = part == 0 ? 2 * H : H; g.N = H; g.K = (int)R; g.batch = D; g.mode = tcg::OUT_ATOMIC_F32; g.a_mn = 1; g.b_mn = 1;
@@ -650,6 +697,10 @@ static int backward_bf16(const bigru_plan& p, const float* params, const float* 
             if (part == 0) TRY(tc_gemm(W + L.gi, (int64_t)D * 3 * H, (int64_t)D * 3 * H, S + L.Yrow[l], (int64_t)D * H, (int64_t)D * H, g, st, KC_TC_GEMM_DWHH));
             else TRY(tc_gemm(W + L.dghn, (int64_t)D * H, (int64_t)D * H, S + L.Yrow[l], (int64_t)D * H, (int64_t)D * H, g, st, KC_TC_GEMM_DWHH));
         }
+        if (h0l)
+            KLAUNCH(KC_MISC, 0.0, 0.0, st, dwhh_h0_kernel<<<dim3((3 * H + 127) / 128, H / DWHH_H0_COLS, D), 128, 0, st>>>(
+                        (const bf16_t*)(W + L.gi), nullptr, (const bf16_t*)(W + L.dghn), nullptr, h0l, grads + p.off_whh(l, 0), p.ld_block(l),
+                        B, T, H, D));
         // 4. dX^T = W_ih^T (both directions concatenated along K = D*3H) x dgi_row^T.  For l > 0 it is written directly in
         //    the blocked layout the next backward scan reads; for layer 0 (caller wants dx) as [F][R] and then re-laid.
         const bool need_dx = l > 0 || dx != nullptr;

@@ -189,27 +189,6 @@ __global__ void __launch_bounds__(256) x3_pack_all_kernel(const X3PackJobs jobs,
     }
 }
 
-// dW_hh[d] += dgh_first^T h0[d]: the first forward step's h_prev is the caller's initial state, which the time-shifted
-// Y operand of the dW_hh GEMM does not contain.  dgh = (hi + lo) of [da_r | da_z] (dgi rows) and da_n * r (dghn rows).
-__global__ void x3_dwhh_h0_kernel(const bf16_t* __restrict__ dgi_hi, const bf16_t* __restrict__ dgi_lo, const bf16_t* __restrict__ dghn_hi,
-                                  const bf16_t* __restrict__ dghn_lo, const float* __restrict__ h0, float* __restrict__ dwhh, int64_t dir_stride,
-                                  int B, int T, int H, int D) {
-    const int d = blockIdx.z;
-    const int q = blockIdx.x * blockDim.x + threadIdx.x;      // gate row of W_hh (0..3H)
-    const int k = blockIdx.y;                                 // column of W_hh
-    if (q >= 3 * H) return;
-    const int64_t t_first = d == 0 ? 0 : T - 1;
-    float acc = 0.f;
-    for (int b = 0; b < B; ++b) {
-        const int64_t row = t_first * B + b;
-        float g;
-        if (q < 2 * H) g = __bfloat162float(dgi_hi[row * D * 3 * H + d * 3 * H + q]) + __bfloat162float(dgi_lo[row * D * 3 * H + d * 3 * H + q]);
-        else g = __bfloat162float(dghn_hi[row * D * H + d * H + q - 2 * H]) + __bfloat162float(dghn_lo[row * D * H + d * H + q - 2 * H]);
-        acc = fmaf(g, h0[((int64_t)d * B + b) * H + k], acc);
-    }
-    dwhh[(int64_t)d * dir_stride + (int64_t)q * H + k] += acc;
-}
-
 // ---------------------------------------------------------------------------------------------------
 // forward
 // ---------------------------------------------------------------------------------------------------
@@ -376,8 +355,8 @@ static int backward_x3(const bigru_plan& p, const float* params, const float* x,
             if (part == 0) TRY(tc_gemm(dgi_hi, (int64_t)D * 3 * H, (int64_t)D * 3 * H, S + L.Yhi[l], (int64_t)D * H, (int64_t)D * H, g, st, KC_TC_GEMM_DWHH, dgi_lo, S + L.Ylo[l]));
             else TRY(tc_gemm(dghn_hi, (int64_t)D * H, (int64_t)D * H, S + L.Yhi[l], (int64_t)D * H, (int64_t)D * H, g, st, KC_TC_GEMM_DWHH, dghn_lo, S + L.Ylo[l]));
         }
-        if (h0)
-            KLAUNCH(KC_MISC, 0.0, 0.0, st, x3_dwhh_h0_kernel<<<dim3((3 * H + 127) / 128, H, D), 128, 0, st>>>(
+        if (h0)   // the first step's h_prev term of dW_hh (dwhh_h0_kernel, path_bf16.cuh)
+            KLAUNCH(KC_MISC, 0.0, 0.0, st, dwhh_h0_kernel<<<dim3((3 * H + 127) / 128, H / DWHH_H0_COLS, D), 128, 0, st>>>(
                         dgi_hi, dgi_lo, dghn_hi, dghn_lo, h0 + (int64_t)l * D * B * H, grads + p.off_whh(l, 0), p.ld_block(l), B, T, H, D));
         const bool need_dx = l > 0 || dx != nullptr;
         if (need_dx) {   // dX^T = W_ih^T (both directions along K = D*3H) x dgi^T

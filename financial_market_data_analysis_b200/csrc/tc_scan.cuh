@@ -129,6 +129,8 @@ struct FwdParams {
     __nv_bfloat16* G;
     __nv_bfloat16* YB;
     float* hn_out;                // [D][B][H] fp32, nullable
+    const float* h0;              // nullable [D][B][H]: initial hidden state of this layer ...
+    const float* gh0;             // ... and its recurrent product W_hh h0 [D][B][3H] (fp32, no bias, formed by the caller): step 0 reads it
     unsigned int* dbg;
     // fused input projection (layer 0, n_features == 64): gi_t = W_ih x_t + b is formed by the same tensor pipe between
     // the recurrent products (it is idle while the epilogue works), giB is not read
@@ -345,9 +347,10 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scan_fwd_kernel(const __grid_c
         const float bhn = p.b_hn[d * H + unit];
         const float bx_r = FX ? p.bfold[d * 3 * H + unit] : 0.f, bx_z = FX ? p.bfold[d * 3 * H + H + unit] : 0.f,
                     bx_n = FX ? p.bfold[d * 3 * H + 2 * H + unit] : 0.f;
+        const bool has_h0 = p.h0 != nullptr && p.gh0 != nullptr;
         float hprev[8];
 #pragma unroll
-        for (int i = 0; i < 8; ++i) hprev[i] = 0.f;
+        for (int i = 0; i < 8; ++i) hprev[i] = has_h0 ? p.h0[((int64_t)d * B + tile * NB + col0 + i) * H + unit] : 0.f;
         // loop-invariant shared-memory offsets: this thread's 8 elements of the h operand tile (inside its 64-unit chunk) and
         // the 16-byte chunk it forwards to the peer
         uint32_t h_off[8];
@@ -415,6 +418,14 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scan_fwd_kernel(const __grid_c
             } else {
 #pragma unroll
                 for (int i = 0; i < 8; ++i) { r8[i] = 0.f; z8[i] = 0.f; an[i] = 0.f; }
+            }
+            if (s == 0 && has_h0) {
+                // step 0 with an initial state: the recurrent product W_hh h0 comes from the caller (no MMA at step 0)
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    const float* gp = p.gh0 + ((int64_t)d * B + tile * NB + col0 + i) * 3 * H + unit;
+                    r8[i] += gp[0]; z8[i] += gp[H]; an[i] += gp[2 * H];
+                }
             }
 #pragma unroll
             for (int i = 0; i < 8; ++i) { r8[i] = sigmoid_fast(gr[i] + r8[i]); z8[i] = sigmoid_fast(gz[i] + z8[i]); }
@@ -551,6 +562,8 @@ struct BwdParams {
     const __nv_bfloat16* G;
     const __nv_bfloat16* YB;        // blocked h (see forward)
     const float* dYB;               // blocked fp32 dY: [block][256][8]   (lower layers)
+    const float* h0;                // nullable [D][B][H]: h_prev of the first forward step
+    float* dh0;                     // nullable [D][B][H]: gradient of the initial hidden state
     // top layer: dY is formed on the fly from the head (biGRU_model.py:111-137): d(concat) = dlogits x lin_w,
     // dY_t[b,u] = davg/T + (argmax_t == t ? dmax : 0), initial carry = d(last hidden); dYB is not read then
     const float* dlogits;           // [B][C] nullable (non-null selects top-layer mode)
@@ -659,7 +672,8 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scan_bwd_kernel(const __grid_c
         // ---- control thread (see forward kernel)
         if (tc::elect_one()) {
             bool ok = true;
-            if (CS > 1 && T > 1) tc::mbar_arrive_expect_tx(&d_full[0], (uint32_t)(CS - 1) * 3 * gate_bytes_mine);
+            const int Tend = T + (p.dh0 ? 1 : 0);          // one more product (no gate math) when d(h0) is wanted
+            if (CS > 1 && Tend > 1) tc::mbar_arrive_expect_tx(&d_full[0], (uint32_t)(CS - 1) * 3 * gate_bytes_mine);
             auto store_tile = [&](int step) {             // dgi / dgh_n rows of time step `step`, this CTA's 128 units
                 const int tt = d == 0 ? T - 1 - step : step;
                 const int row = tt * B + tile * NB;
@@ -682,7 +696,7 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scan_bwd_kernel(const __grid_c
             const uint64_t d_loc0 = tc::umma_desc_k_sw128(db0 + (uint32_t)c * gate_bytes_mine);
             const uint64_t d_rem0 = tc::umma_desc_k_sw128(db0 + (uint32_t)(1 - (int)c) * gate_bytes_mine);
             constexpr uint64_t BUF_DESC = (uint64_t)((KC3 * H_CHUNK) >> 4);
-            for (int s = 1; s < T; ++s) {
+            for (int s = 1; s < Tend; ++s) {
                 const int pb = (s - 1) & 1;
                 if (ok) ok = tc::mbar_wait(epi_done, (s - 1) & 1, p.dbg, 0x700 + (s & 0xff));
                 SCAN_TS(0);
@@ -692,7 +706,7 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scan_bwd_kernel(const __grid_c
                     SCAN_TS(1);
                     if (ok) ok = tc::mbar_wait(&d_full[pb], ((s - 1) >> 1) & 1, p.dbg, 0x800 + (s & 0xff));
                     SCAN_TS(2);
-                    if (s + 1 < T) tc::mbar_arrive_expect_tx(&d_full[s & 1], (uint32_t)(CS - 1) * 3 * gate_bytes_mine);
+                    if (s + 1 < Tend) tc::mbar_arrive_expect_tx(&d_full[s & 1], (uint32_t)(CS - 1) * 3 * gate_bytes_mine);
                     tc::tcgen05_fence_after();
                     bwd_issue_group<H, MYCH, false>(tmem, a_rem, d_rem0 + (pb ? BUF_DESC : 0));
                 } else {
@@ -704,9 +718,11 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scan_bwd_kernel(const __grid_c
                 if (ok) ok = tc::mbar_wait(st_done, (s - 1) & 1, p.dbg, 0xa00 + (s & 0xff));
                 store_tile(s - 1);
             }
-            if (ok) ok = tc::mbar_wait(epi_done, (T - 1) & 1, p.dbg, 0x700);
-            if (ok) ok = tc::mbar_wait(st_done, (T - 1) & 1, p.dbg, 0xa00);
-            store_tile(T - 1);
+            if (Tend == T) {
+                if (ok) ok = tc::mbar_wait(epi_done, (T - 1) & 1, p.dbg, 0x700);
+                if (ok) ok = tc::mbar_wait(st_done, (T - 1) & 1, p.dbg, 0xa00);
+                store_tile(T - 1);
+            }
             tc::tma_store_wait_all();
         }
     } else if (warp < EPI_WARPS) {
@@ -745,6 +761,7 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scan_bwd_kernel(const __grid_c
         const int kc_u = unit >> 6;
         const int gu = (int)c * UNITS + q * 32 + (lane >> 3) * 8;
         const uint32_t fwd_off = (uint32_t)(gu >> 6) * H_CHUNK + tc::sw128_offset(col0 + (lane & 7), gu & 63);
+        const int Tend = T + (p.dh0 ? 1 : 0);              // the dgh of the last step also feeds d(h0) (control thread)
         bool ok = true;
         for (int s = 0; s < T; ++s) {
             const int t = d == 0 ? T - 1 - s : s;
@@ -780,6 +797,10 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scan_bwd_kernel(const __grid_c
                 t8 = reinterpret_cast<const __nv_bfloat16*>(&uh);
 #pragma unroll
                 for (int i = 0; i < 8; ++i) vhp[i] = __bfloat162float(t8[i]);
+                if (first && p.h0) {                        // the caller's initial state, in fp32
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) vhp[i] = p.h0[((int64_t)d * B + tile * NB + col0 + i) * H + unit];
+                }
                 vdy[0] = a.x; vdy[1] = a.y; vdy[2] = a.z; vdy[3] = a.w; vdy[4] = b.x; vdy[5] = b.y; vdy[6] = b.z; vdy[7] = b.w;
                 if (top) {                                  // dY_t = davg / T + (argmax_t == t ? dmax : 0)
 #pragma unroll
@@ -840,7 +861,7 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scan_bwd_kernel(const __grid_c
             // the local arrival; the n-gate tile (TMA store only) and the bias sums follow, off the chain
             if (tid == 0) SCAN_TS(9);
             tc::tcgen05_fence_before();
-            if (CS > 1 && s + 1 < T) {
+            if (CS > 1 && s + 1 < Tend) {
                 __syncwarp();
                 const uint32_t rbar = tc::mapa_u32(tc::smem_u32(&d_full[buf]), 1u - c);
 #pragma unroll
@@ -873,6 +894,16 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scan_bwd_kernel(const __grid_c
         float* dbh = p.db_hh + (int64_t)d * p.dir_stride;
         atomicAdd(dbi + unit, sb_r); atomicAdd(dbi + H + unit, sb_z); atomicAdd(dbi + 2 * H + unit, sb_n);
         atomicAdd(dbh + unit, sb_r); atomicAdd(dbh + H + unit, sb_z); atomicAdd(dbh + 2 * H + unit, sb_nr);
+        if (p.dh0) {
+            // gradient of the initial hidden state = z-carry of the last step + W_hh^T dgh of the last step (one more product)
+            float acc[8];
+            if (ok) ok = tc::mbar_wait(mma_done, (T - 1) & 1, p.dbg, 0x900);
+            tc::tcgen05_fence_after();
+            tmem_ld8(tmem + ((uint32_t)(q * 32) << 16) + col0, acc);
+            tc::tmem_ld_wait();
+#pragma unroll
+            for (int i = 0; i < 8; ++i) p.dh0[((int64_t)d * B + tile * NB + col0 + i) * H + unit] = dhz[i] + acc[i];
+        }
     }
     tc::tcgen05_fence_before();
     __syncthreads();

@@ -82,6 +82,8 @@ struct FwdParams {
     __nv_bfloat16* GW;
     __nv_bfloat16* YBW;
     float* hn_out;                // nullable [D][B][H]
+    const float* h0;              // nullable [D][B][H]: initial hidden state of this layer ...
+    const float* gh0;             // ... and its recurrent product W_hh h0 [D][B][3H] (fp32, no bias, formed by the caller): step 0 reads it
     __nv_bfloat16* Yrow;          // [R][D*H]
     unsigned int* dbg;
     CUtensorMap tmY;              // box 64 x 32 (filled by launch_fwd)
@@ -256,9 +258,10 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scanw_fwd_kernel(const __grid_
         const int c0 = 16 * half + 8 * part;               // == 8 * (warp >> 1)
         const int tid = threadIdx.x;
         const float bhn = p.b_hn[d * H + unit];
+        const bool has_h0 = p.h0 != nullptr && p.gh0 != nullptr;
         float hprev[8];
 #pragma unroll
-        for (int i = 0; i < 8; ++i) hprev[i] = 0.f;
+        for (int i = 0; i < 8; ++i) hprev[i] = has_h0 ? p.h0[((int64_t)d * B + tile * NB + c0 + i) * H + unit] : 0.f;
         uint32_t h_off[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) h_off[i] = c * H_CHUNK + tc::sw128_offset(c0 + i, j);
@@ -316,6 +319,13 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scanw_fwd_kernel(const __grid_
                     an[0] = n0.x; an[1] = n0.y; an[2] = n0.z; an[3] = n0.w; an[4] = n1.x; an[5] = n1.y; an[6] = n1.z; an[7] = n1.w;
 #pragma unroll
                     for (int i = 0; i < 8; ++i) az[i] = va[8 + i];
+                }
+            } else if (has_h0) {
+                // step 0 with an initial state: the recurrent product W_hh h0 comes from the caller (no MMA at step 0)
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    const float* gp = p.gh0 + ((int64_t)d * B + tile * NB + c0 + i) * 3 * H + unit;
+                    ar[i] = gp[0]; az[i] = gp[H]; an[i] = gp[2 * H];
                 }
             } else {
 #pragma unroll
@@ -412,6 +422,8 @@ struct BwdParams {
     const __nv_bfloat16* GW;
     const __nv_bfloat16* YBW;
     const float* dYBW;              // lower layers
+    const float* h0;                // nullable [D][B][H]: h_prev of the first forward step
+    float* dh0;                     // nullable [D][B][H]: gradient of the initial hidden state
     const float* dlogits;           // top layer: dL/dlogits [B][C], head weights and the max-pool arg-max (see tc_scan.cuh)
     const float* lin_w;
     const int* arg;
@@ -524,7 +536,8 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scanw_bwd_kernel(const __grid_
                 tc::tma_store_commit();
             };
             const uint32_t db0 = tc::smem_u32(sD);
-            for (int s = 1; s < T; ++s) {
+            const int Tend = T + (p.dh0 ? 1 : 0);          // one more product (no gate math) when d(h0) is wanted
+            for (int s = 1; s < Tend; ++s) {
                 const int pb = (s - 1) & 1;
                 if (ok) ok = tc::mbar_wait(epi_done, (s - 1) & 1, p.dbg, 0x4700 + (s & 0xff));
                 tc::tcgen05_fence_after();
@@ -542,9 +555,11 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scanw_bwd_kernel(const __grid_
                 if (ok) ok = tc::mbar_wait(st_done, (s - 1) & 1, p.dbg, 0x4a00 + (s & 0xff));
                 store_tile(s - 1);
             }
-            if (ok) ok = tc::mbar_wait(epi_done, (T - 1) & 1, p.dbg, 0x4700);
-            if (ok) ok = tc::mbar_wait(st_done, (T - 1) & 1, p.dbg, 0x4a00);
-            store_tile(T - 1);
+            if (Tend == T) {
+                if (ok) ok = tc::mbar_wait(epi_done, (T - 1) & 1, p.dbg, 0x4700);
+                if (ok) ok = tc::mbar_wait(st_done, (T - 1) & 1, p.dbg, 0x4a00);
+                store_tile(T - 1);
+            }
             tc::tma_store_wait_all();
         }
     } else {
@@ -640,6 +655,10 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scanw_bwd_kernel(const __grid_
                 if (!first) uh = tc::lds_u4(gp + G_BLOCK);
                 if (!top) { y0 = tc::lds_f4(sIn_u + (uint32_t)st * BWD_STAGE + G_BLOCK + YB_BLOCK + 32u * tid); y1 = tc::lds_f4(sIn_u + (uint32_t)st * BWD_STAGE + G_BLOCK + YB_BLOCK + 32u * tid + 16); }
                 unpack8(u0, vr); unpack8(u1, vz); unpack8(u2, vn); unpack8(u3, vhn); unpack8(uh, vhp);
+                if (first && p.h0) {                        // the caller's initial state, in fp32
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) vhp[i] = p.h0[((int64_t)d * B + tile * NB + c0 + i) * H + unit];
+                }
                 vdy[0] = y0.x; vdy[1] = y0.y; vdy[2] = y0.z; vdy[3] = y0.w; vdy[4] = y1.x; vdy[5] = y1.y; vdy[6] = y1.z; vdy[7] = y1.w;
                 if (top) {
 #pragma unroll
@@ -695,6 +714,13 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scanw_bwd_kernel(const __grid_
         float* dbh = p.db_hh + (int64_t)d * p.dir_stride;
         atomicAdd(dbi + unit, sb_r); atomicAdd(dbi + H + unit, sb_z); atomicAdd(dbi + 2 * H + unit, sb_n);
         atomicAdd(dbh + unit, sb_r); atomicAdd(dbh + H + unit, sb_z); atomicAdd(dbh + 2 * H + unit, sb_nr);
+        if (p.dh0) {
+            // gradient of the initial hidden state = z-carry of the last step + W_hh^T dgh of the last step (one more product)
+            float acc[8];
+            reduce_partials(T, acc);
+#pragma unroll
+            for (int i = 0; i < 8; ++i) p.dh0[((int64_t)d * B + tile * NB + c0 + i) * H + unit] = dhz[i] + acc[i];
+        }
     }
     tc::tcgen05_fence_before();
     __syncthreads();
@@ -805,7 +831,8 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scanw_bwd2_kernel(const __grid
                 tc::tma_store_commit();
             };
             const uint32_t db0 = tc::smem_u32(sD);
-            for (int s = 1; s < T; ++s) {
+            const int Tend = T + (p.dh0 ? 1 : 0);          // one more product (no gate math) when d(h0) is wanted
+            for (int s = 1; s < Tend; ++s) {
                 const int pb = (s - 1) & 1;
 #pragma unroll
                 for (int sub = 0; sub < 2; ++sub) {
@@ -827,10 +854,12 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scanw_bwd2_kernel(const __grid
                     store_tile(sub, s - 1);
                 }
             }
-            for (int sub = 0; sub < 2; ++sub) {
-                if (ok) ok = tc::mbar_wait(&epi_done[sub], (T - 1) & 1, p.dbg, 0x4700);
-                if (ok) ok = tc::mbar_wait(&st_done[sub], (T - 1) & 1, p.dbg, 0x4a00);
-                store_tile(sub, T - 1);
+            if (Tend == T) {
+                for (int sub = 0; sub < 2; ++sub) {
+                    if (ok) ok = tc::mbar_wait(&epi_done[sub], (T - 1) & 1, p.dbg, 0x4700);
+                    if (ok) ok = tc::mbar_wait(&st_done[sub], (T - 1) & 1, p.dbg, 0x4a00);
+                    store_tile(sub, T - 1);
+                }
             }
             tc::tma_store_wait_all();
         }
@@ -928,6 +957,10 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scanw_bwd2_kernel(const __grid
                 if (!first) uh = tc::lds_u4(gp + G_BLOCK);
                 if (!top) { y0 = tc::lds_f4(sIn_u + (uint32_t)st * BWD_STAGE + G_BLOCK + YB_BLOCK + 32u * tid); y1 = tc::lds_f4(sIn_u + (uint32_t)st * BWD_STAGE + G_BLOCK + YB_BLOCK + 32u * tid + 16); }
                 unpack8(u0, vr); unpack8(u1, vz); unpack8(u2, vn); unpack8(u3, vhn); unpack8(uh, vhp);
+                if (first && p.h0) {                        // the caller's initial state, in fp32
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) vhp[i] = p.h0[((int64_t)d * B + tile * NB + c0 + i) * H + unit];
+                }
                 vdy[0] = y0.x; vdy[1] = y0.y; vdy[2] = y0.z; vdy[3] = y0.w; vdy[4] = y1.x; vdy[5] = y1.y; vdy[6] = y1.z; vdy[7] = y1.w;
                 if (top) {
 #pragma unroll
@@ -983,6 +1016,13 @@ __global__ void __launch_bounds__(THREADS, 1) gru_scanw_bwd2_kernel(const __grid
         float* dbh = p.db_hh + (int64_t)d * p.dir_stride;
         atomicAdd(dbi + unit, sb_r); atomicAdd(dbi + H + unit, sb_z); atomicAdd(dbi + 2 * H + unit, sb_n);
         atomicAdd(dbh + unit, sb_r); atomicAdd(dbh + H + unit, sb_z); atomicAdd(dbh + 2 * H + unit, sb_nr);
+        if (p.dh0) {
+            // gradient of the initial hidden state = z-carry of the last step + W_hh^T dgh of the last step (one more product)
+            float acc[8];
+            reduce_partials(T, acc);
+#pragma unroll
+            for (int i = 0; i < 8; ++i) p.dh0[((int64_t)d * B + tile * NB + c0 + i) * H + unit] = dhz[i] + acc[i];
+        }
     }
     tc::tcgen05_fence_before();
     __syncthreads();

@@ -40,7 +40,8 @@ extern "C" {
 #define BIGRU_PREC_FP32 0          /* fp32 FFMA path: exact, any shape (<=1e-4 rel on logits) */
 #define BIGRU_PREC_BF16 1          /* bf16 operands on tcgen05 tensor cores, fp32 accumulate/state.
                                       hidden_size 128 or 256 with batch % 16 == 0, hidden_size 512 with batch % 32 == 0
-                                      (BASELINE.json configs[4]); no initial hidden state */
+                                      (BASELINE.json configs[4]); d_h0 / d_dh0 are supported (W_hh h0 is formed in fp32,
+                                      h0 enters the gate math of the first step and dW_hh in fp32) */
 #define BIGRU_PREC_BF16X3 2        /* fp32-class on tensor cores: (hi, lo) bf16 operand pairs, 3-4 products per term,
                                       fp32 accumulate / gate math / stash; meets the 1e-4 logit tolerance at tensor-core speed.
                                       hidden_size 128 or 256, batch % 32 == 0.
