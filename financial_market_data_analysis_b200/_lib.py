@@ -44,6 +44,9 @@ SIGNATURES = {
     "bigru_forward_windows": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _f, _i, _i, _u64, _vp, _vp, _vp, _vp, _vp]),
     "bigru_chunk_minmax": (_i, [_vp, _i64, _i, _i64, _i64, _vp, _vp, _vp]),
     "bigru_infer_window": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "bigru_infer_cluster_workspace_bytes": (_i, [_i, _i, _i, _i, _i, _i, C.POINTER(C.c_size_t)]),
+    "bigru_infer_cluster": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "bigru_infer_cluster_geometry": (_i, [_i, _i, _i, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),
     "bigru_window_features": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, C.POINTER(_i), _i, C.POINTER(_i), _i, C.POINTER(_i), _i, _i, _f, _i,
                                    _f, _f, _vp, _vp, C.POINTER(_i), _vp]),
     "bigru_launch_count": (C.c_longlong, []),

@@ -5,7 +5,9 @@
 #include "path_x3.cuh"
 #include "features.cuh"
 #include "infer_small.cuh"
+#include "infer_cluster.cuh"
 
+#include <cstdlib>
 #include <cstring>
 #include <new>
 
@@ -475,6 +477,173 @@ extern "C" int bigru_infer_window(const float* d_params, const float* d_x, const
     const int threads = std::max(32, ((DH + 31) / 32) * 32);
     KLAUNCH(KC_MISC, 0.0, 0.0, (cudaStream_t)stream,
             infer_window_kernel<<<B, threads, smem, (cudaStream_t)stream>>>(d_params, d_x, d_xmin, d_xmax, T, F, H, L, C, D, d_logits, d_probs));
+    return BIGRU_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// cluster-resident live inference (csrc/infer_cluster.cuh).  Workspace in floats, each region 256-byte aligned:
+// normalised input [B*T*F] | gi [D][B*T][3H] | layer output Y [B][T][D*H] (reused by every layer: a layer's projection
+// has consumed its input before its scan overwrites it).
+// ------------------------------------------------------------------------------------------
+struct InferWork { int64_t xn, gi, y, total; };
+static InferWork infer_work_layout(int B, int T, int F, int H, int D) {
+    auto al = [](int64_t n) { return (n + 63) / 64 * 64; };
+    const int64_t BT = (int64_t)B * T;
+    InferWork w{};
+    w.xn = 0;
+    w.gi = w.xn + al(BT * F);
+    w.y = w.gi + al((int64_t)D * BT * 3 * H);
+    w.total = w.y + al(BT * D * H);
+    return w;
+}
+
+static bool infer_cluster_shape_ok(int B, int T, int F, int H, int L, int C) {
+    return B > 0 && T > 0 && F > 0 && H > 0 && L > 0 && C > 0;
+}
+
+extern "C" int bigru_infer_cluster_workspace_bytes(int B, int T, int F, int H, int L, int bidirectional, size_t* bytes) {
+    if (!bytes || !infer_cluster_shape_ok(B, T, F, H, L, 1)) {
+        bigru_set_error("infer_cluster_workspace_bytes: bad argument");
+        return BIGRU_ERR_ARG;
+    }
+    *bytes = (size_t)infer_work_layout(B, T, F, H, bidirectional ? 2 : 1).total * sizeof(float);
+    return BIGRU_OK;
+}
+
+// Cluster geometry: U units per CTA (a multiple of 4, at most 32), NC = ceil(H / U) CTAs.  The per-step time is bound by the
+// shared-memory reads of the W_hh slice (3*U*Hp*4 bytes per CTA), so the widest cluster wins: up to 16 CTAs
+// (non-portable) where the device grants them, else 8.  BIGRU_INFER_CLUSTER_CTAS (8 or 16) caps it for measurement.
+// G windows per cluster: the smallest power of two <= 4 that covers B (capped by shared memory; G = 8 spills registers).
+struct InferGeo { int NC, U, Hp, G; size_t smem; };
+static InferGeo infer_geometry(int B, int H, int max_nc) {
+    InferGeo g{};
+    g.U = (int)((cdiv64(H, max_nc) + 3) / 4 * 4);
+    g.NC = (int)cdiv64(H, g.U);
+    g.Hp = g.NC * g.U;
+    g.G = 1;
+    while (g.G < 4 && g.G < B) g.G *= 2;
+    while (g.G > 1 && icl::scan_smem_bytes(g.U, g.Hp, g.G) > 227 * 1024) g.G /= 2;
+    g.smem = icl::scan_smem_bytes(g.U, g.Hp, g.G);
+    return g;
+}
+
+template <int G>
+static int infer_scan_launch(const InferGeo& geo, int ngroups, int D, const float* gi, const float* w_hh, const float* b_hh,
+                             int64_t dir_stride, float* Y, int B, int T, int H, cudaStream_t st, bool probe, int* max_clusters) {
+    auto kern = icl::infer_cluster_scan_kernel<G>;
+    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)geo.smem));
+    if (geo.NC > 8) CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(geo.NC, ngroups, D);
+    cfg.blockDim = dim3(icl::kThreads);
+    cfg.dynamicSmemBytes = geo.smem;
+    cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = geo.NC; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    if (probe) {
+        int n = 0;
+        cudaError_t e = cudaOccupancyMaxActiveClusters(&n, kern, &cfg);
+        if (e != cudaSuccess) { cudaGetLastError(); n = 0; }
+        *max_clusters = n;
+        return BIGRU_OK;
+    }
+    KLAUNCH(KC_INFER, 0.0, 0.0, st, CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, gi, w_hh, b_hh, dir_stride, Y, B, T, H, D, geo.U)));
+    return BIGRU_OK;
+}
+
+static int infer_scan_dispatch(const InferGeo& geo, int ngroups, int D, const float* gi, const float* w_hh, const float* b_hh,
+                               int64_t dir_stride, float* Y, int B, int T, int H, cudaStream_t st, bool probe, int* max_clusters) {
+    switch (geo.G) {
+        case 1: return infer_scan_launch<1>(geo, ngroups, D, gi, w_hh, b_hh, dir_stride, Y, B, T, H, st, probe, max_clusters);
+        case 2: return infer_scan_launch<2>(geo, ngroups, D, gi, w_hh, b_hh, dir_stride, Y, B, T, H, st, probe, max_clusters);
+        default: return infer_scan_launch<4>(geo, ngroups, D, gi, w_hh, b_hh, dir_stride, Y, B, T, H, st, probe, max_clusters);
+    }
+}
+
+// the widest cluster the device grants at this shared-memory size (opt-ins set on every call); *granted is
+// cudaOccupancyMaxActiveClusters of the chosen launch
+static int infer_pick_geometry(int B, int H, int D, InferGeo* out, int* granted) {
+    if (H > icl::kMaxHidden) {
+        bigru_set_error("infer_cluster: hidden size %d above %d (16 CTAs x 32 units) is not supported", H, icl::kMaxHidden);
+        return BIGRU_ERR_UNSUPPORTED;
+    }
+    int cap = icl::kMaxCluster;
+    if (const char* e = getenv("BIGRU_INFER_CLUSTER_CTAS")) cap = atoi(e) == 8 ? 8 : icl::kMaxCluster;
+    InferGeo geo = infer_geometry(B, H, cap);
+    *granted = 0;
+    TRY(infer_scan_dispatch(geo, (int)cdiv64(B, geo.G), D, nullptr, nullptr, nullptr, 0, nullptr, B, 1, H, nullptr, true, granted));
+    if (*granted <= 0 && geo.NC > 8) {
+        const int nc16 = geo.NC;
+        geo = infer_geometry(B, H, 8);
+        if (geo.U > icl::kMaxUnits) {
+            bigru_set_error("infer_cluster: hidden size %d needs a %d-CTA cluster, which this device does not grant; "
+                            "8-CTA clusters hold H <= %d", H, nc16, 8 * icl::kMaxUnits);
+            return BIGRU_ERR_UNSUPPORTED;
+        }
+        TRY(infer_scan_dispatch(geo, (int)cdiv64(B, geo.G), D, nullptr, nullptr, nullptr, 0, nullptr, B, 1, H, nullptr, true, granted));
+    }
+    if (*granted <= 0) {
+        bigru_set_error("infer_cluster: the device grants no %d-CTA cluster with %zu bytes of shared memory per CTA", geo.NC, geo.smem);
+        return BIGRU_ERR_UNSUPPORTED;
+    }
+    *out = geo;
+    return BIGRU_OK;
+}
+
+extern "C" int bigru_infer_cluster_geometry(int B, int H, int bidirectional, int* cluster_ctas, int* units_per_cta,
+                                            int* windows_per_cluster, int* max_active_clusters) {
+    if (B <= 0 || H <= 0 || !cluster_ctas || !units_per_cta || !windows_per_cluster || !max_active_clusters) {
+        bigru_set_error("infer_cluster_geometry: bad argument");
+        return BIGRU_ERR_ARG;
+    }
+    InferGeo geo;
+    TRY(infer_pick_geometry(B, H, bidirectional ? 2 : 1, &geo, max_active_clusters));
+    *cluster_ctas = geo.NC; *units_per_cta = geo.U; *windows_per_cluster = geo.G;
+    return BIGRU_OK;
+}
+
+extern "C" int bigru_infer_cluster(const float* d_params, const float* d_x, const float* d_xmin, const float* d_xmax, int B, int T,
+                                   int F, int H, int L, int C, int bidirectional, void* d_work, float* d_logits, float* d_probs,
+                                   void* stream) {
+    if (!d_params || !d_x || !d_work || !d_logits || !infer_cluster_shape_ok(B, T, F, H, L, C) || L > 16 ||
+        ((d_xmin == nullptr) != (d_xmax == nullptr)) || ((uintptr_t)d_work & 15)) {
+        bigru_set_error("infer_cluster: bad argument");
+        return BIGRU_ERR_ARG;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int D = bidirectional ? 2 : 1;
+    InferGeo geo;
+    int granted = 0;
+    TRY(infer_pick_geometry(B, H, D, &geo, &granted));
+    const int ngroups = (int)cdiv64(B, geo.G);
+    bigru_plan p{};
+    p.B = B; p.T = T; p.F = F; p.H = H; p.L = L; p.C = C; p.D = D;
+    const InferWork w = infer_work_layout(B, T, F, H, D);
+    float* work = (float*)d_work;
+    const int64_t BT = (int64_t)B * T;
+    const float* inp = d_x;
+    if (d_xmin) {
+        // (x - min) / (max - min) of every row: the window gather over B*T consecutive rows
+        float* xn = work + w.xn;
+        const unsigned blocks = (unsigned)std::min<int64_t>(cdiv64(BT * F, 256), 148 * 8);
+        KLAUNCH(KC_GATHER, 0.0, 8.0 * BT * F, st, window_gather_kernel<1><<<blocks, 256, 0, st>>>(d_x, d_xmin, d_xmax, 0, 1, (int)BT, F, xn));
+        inp = xn;
+    }
+    float* Y = work + w.y;
+    for (int l = 0; l < L; ++l) {
+        const int I = (int)p.in_size(l);
+        GemmArgs g = gemm_args(inp, d_params + p.off_wih(l, 0), work + w.gi, (int)BT, 3 * H, I, I, 1, I, 1, 3 * H);
+        g.bias = d_params + p.off_bih(l, 0);
+        g.batch = D; g.zA = 0; g.zB = p.ld_block(l); g.zBias = p.ld_block(l); g.zC = BT * 3 * H;
+        TRY(sgemm_launch(g, st));
+        TRY(infer_scan_dispatch(geo, ngroups, D, work + w.gi, d_params + p.off_whh(l, 0), d_params + p.off_bhh(l, 0), p.ld_block(l), Y,
+                                B, T, H, st, false, nullptr));
+        inp = Y;
+    }
+    KLAUNCH(KC_HEAD, 0.0, 0.0, st,
+            icl::infer_head_kernel<<<B, 128, 3 * H * sizeof(float), st>>>(Y, d_params + p.off_linw(), T, H, C, D, d_logits, d_probs));
     return BIGRU_OK;
 }
 

@@ -9,11 +9,11 @@
 
 enum KClass {
     KC_SGEMM = 0, KC_GATES_FWD, KC_GATES_BWD, KC_HEAD, KC_LOSS, KC_OPTIM, KC_GATHER, KC_MISC,
-    KC_TC_GEMM, KC_TC_SCAN_FWD, KC_TC_SCAN_BWD, KC_PACK, KC_TC_GEMM_DX, KC_TC_GEMM_DWIH, KC_TC_GEMM_DWHH, KC_COUNT
+    KC_TC_GEMM, KC_TC_SCAN_FWD, KC_TC_SCAN_BWD, KC_PACK, KC_TC_GEMM_DX, KC_TC_GEMM_DWIH, KC_TC_GEMM_DWHH, KC_INFER, KC_COUNT
 };
 static const char* const kKClassNames[KC_COUNT] = {
     "sgemm_f32", "gru_gates_fwd", "gru_gates_bwd", "head", "loss", "clip_adam", "window_gather", "misc",
-    "tc_gemm_proj", "tc_gru_scan_fwd", "tc_gru_scan_bwd", "pack_bf16", "tc_gemm_dx", "tc_gemm_dwih", "tc_gemm_dwhh"};
+    "tc_gemm_proj", "tc_gru_scan_fwd", "tc_gru_scan_bwd", "pack_bf16", "tc_gemm_dx", "tc_gemm_dwih", "tc_gemm_dwhh", "infer_cluster_scan"};
 
 struct ProfRec { int cls; double flops, bytes; cudaEvent_t a, b; };
 struct Profiler {

@@ -5,9 +5,10 @@ spatial_dropout=False, bidirectional=True)`` (``:73-88``), loads ``model_params.
 ``norm_params`` (``:110-122``), and for every Kafka message fetches one window of ``window=5`` rows, normalises it
 ``(x - min) / (max - min)`` (``:170``), runs ``model.forward`` in eval mode (``:178``), applies a sigmoid (``:181``) and
 reports the labels above ``prob_threshold`` (``:186-193``).  The Kafka consumer / producer and the MySQL cursor stay the
-reference's own; :class:`LivePredictor` is the part between "rows fetched" and "dict to send", and does it in **one
-kernel launch** (``bigru_infer_window``: normalisation + GRU + pooling head + Linear + sigmoid) instead of the
-step-by-step launches of the training path.  There is no CPU fallback."""
+reference's own; :class:`LivePredictor` is the part between "rows fetched" and "dict to send".  Small models (the
+shipped checkpoint) run in **one kernel launch** (``bigru_infer_window``: normalisation + GRU + pooling head + Linear +
+sigmoid, one CTA per window); full-size models (long windows, hidden sizes up to 512) run on ``bigru_infer_cluster``
+(one SGEMM and one cluster-resident scan per layer, then the head).  There is no CPU fallback."""
 from __future__ import annotations
 
 import pickle
@@ -21,14 +22,28 @@ from .biGRU_model import BiGRU
 
 Y_FIELDS = "up1, up2, down1, down2".split(", ")        # predict.py:33
 
+# bigru_infer_window (one CTA per window, one launch) is used where it accepts the shape and hidden_size <=
+# SINGLE_CTA_MAX_HIDDEN; otherwise bigru_infer_cluster (2L+1 launches).  The bound keeps the shipped (H 8) and notebook
+# (H 32) models on one launch.  The crossover is not measured yet: tools/bench_live_predictor.py measures it (DESIGN §5.7b).
+SINGLE_CTA_MAX_HIDDEN = 32
+
+
+def checkpoint_shape(state):
+    """(hidden_size, n_layers) of a BiGRU state dict: the columns of ``gru.weight_hh_l0`` and the number of
+    ``gru.weight_ih_l{k}`` keys."""
+    hidden = int(state["gru.weight_hh_l0"].shape[1])
+    layers = sum(1 for k in state if k.startswith("gru.weight_ih_l") and not k.endswith("_reverse"))
+    return hidden, layers
+
 
 class LivePredictor:
     def __init__(self, model_params="model_params.pt", norm_params="norm_params", n_features=None, y_fields=Y_FIELDS,
-                 window=5, hidden_size=8, n_layers=1, clip=50, dropout=0.2, learning_rate=0.001, spatial_dropout=False,
+                 window=5, hidden_size=None, n_layers=None, clip=50, dropout=0.2, learning_rate=0.001, spatial_dropout=False,
                  prob_threshold=0.5, device="cuda"):
         """``model_params``: path to the checkpoint or a state_dict; ``norm_params``: path to the pickle written by
         ``MySQLChunkLoader`` (``sql_pytorch_dataloader.py:146-153``), the dict itself (name -> {"MIN", "MAX"}), a
-        ``(min, max)`` pair of arrays, or ``None`` for already normalised windows.  Defaults as ``predict.py:73-83``."""
+        ``(min, max)`` pair of arrays, or ``None`` for already normalised windows.  ``hidden_size`` / ``n_layers`` default to
+        the checkpoint's own shape (the shipped one: 8 and 1); other defaults as ``predict.py:73-83``."""
         self.window, self.prob_threshold, self.y_fields = int(window), float(prob_threshold), list(y_fields)
         if isinstance(norm_params, str):
             with open(norm_params, "rb") as fh:
@@ -47,6 +62,10 @@ class LivePredictor:
         dev = torch.device(device)
         if dev.type != "cuda":
             raise RuntimeError("LivePredictor runs on the GPU only (no CPU fallback)")
+        if hidden_size is None or n_layers is None:
+            ck_hidden, ck_layers = checkpoint_shape(state)
+            hidden_size = ck_hidden if hidden_size is None else int(hidden_size)
+            n_layers = ck_layers if n_layers is None else int(n_layers)
         model = BiGRU(hidden_size, self.n_features, len(self.y_fields), n_layers, clip, dropout, spatial_dropout, bidirectional=True,
                       precision="fp32")
         model.to(dev)                                                      # predict.py:90-91
@@ -65,9 +84,10 @@ class LivePredictor:
         self._logits = torch.empty((1, C), dtype=torch.float32, device=dev)
         self._probs = torch.empty((1, C), dtype=torch.float32, device=dev)
         self._host = torch.empty((2, C), dtype=torch.float32).pin_memory()
+        self._work = torch.empty(0, dtype=torch.float32, device=dev)     # bigru_infer_cluster workspace, grown as needed
 
     def forward_windows(self, windows):
-        """Raw (un-normalised) windows [B, window, n_features] -> (logits, probabilities) on the device, one launch."""
+        """Raw (un-normalised) windows [B, window, n_features] -> (logits, probabilities) on the device."""
         m = self.model
         x = torch.as_tensor(windows, dtype=torch.float32).to(self.device, non_blocking=True).contiguous()
         if x.dim() == 2:
@@ -78,11 +98,33 @@ class LivePredictor:
         logits = self._logits if B == 1 else torch.empty((B, len(self.y_fields)), dtype=torch.float32, device=self.device)
         probs = self._probs if B == 1 else torch.empty_like(logits)
         lib = _lib.load()
+        H, L, C, bi = m.hidden_size, m.n_layers, m.output_size, 1 if m.bidirectional else 0
+        xmin, xmax = _lib.ptr(self.x_min), _lib.ptr(self.x_max)
         with torch.cuda.device(self.device):
-            _lib.check(lib.bigru_infer_window(_lib.ptr(m.flat_parameters()), _lib.ptr(x), _lib.ptr(self.x_min) if self.x_min is not None else None,
-                                              _lib.ptr(self.x_max) if self.x_max is not None else None, B, T, self.n_features, m.hidden_size,
-                                              m.n_layers, m.output_size, 1 if m.bidirectional else 0, _lib.ptr(logits), _lib.ptr(probs),
-                                              torch.cuda.current_stream(self.device).cuda_stream), "bigru_infer_window")
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            params = m.flat_parameters()
+            rc = _lib.ERR_UNSUPPORTED
+            if H <= SINGLE_CTA_MAX_HIDDEN:
+                rc = lib.bigru_infer_window(_lib.ptr(params), _lib.ptr(x), xmin, xmax, B, T, self.n_features, H, L, C, bi,
+                                            _lib.ptr(logits), _lib.ptr(probs), stream)
+                if rc != _lib.ERR_UNSUPPORTED:
+                    _lib.check(rc, "bigru_infer_window")
+            if rc == _lib.ERR_UNSUPPORTED:
+                nbytes = _lib.C.c_size_t()
+                _lib.check(lib.bigru_infer_cluster_workspace_bytes(B, T, self.n_features, H, L, bi, _lib.C.byref(nbytes)),
+                           "bigru_infer_cluster_workspace_bytes")
+                if self._work.numel() * 4 < nbytes.value:
+                    self._work = torch.empty((nbytes.value + 3) // 4, dtype=torch.float32, device=self.device)
+                rc = lib.bigru_infer_cluster(_lib.ptr(params), _lib.ptr(x), xmin, xmax, B, T, self.n_features, H, L, C, bi,
+                                             _lib.ptr(self._work), _lib.ptr(logits), _lib.ptr(probs), stream)
+                if rc != _lib.ERR_UNSUPPORTED:
+                    _lib.check(rc, "bigru_infer_cluster")
+            if rc == _lib.ERR_UNSUPPORTED:
+                # neither live kernel takes the shape: the model's own fp32 forward (eval mode, no dropout)
+                xn = x if self.x_min is None else (x - self.x_min) / (self.x_max - self.x_min)
+                with torch.no_grad():
+                    logits.copy_(m(xn))
+                torch.sigmoid(logits, out=probs)
         return logits, probs
 
     def predict(self, input_data, timestamp_str=None):

@@ -176,6 +176,23 @@ int  bigru_window_features(const float* d_close, const float* d_high, const floa
 int  bigru_infer_window(const float* d_params, const float* d_x, const float* d_xmin, const float* d_xmax, int B, int T,
                         int F, int H, int L, int C, int bidirectional, float* d_logits, float* d_probs, void* stream);
 
+/* --- The live predictor's forward for full-size models (any T, F, L; H <= 512): same inputs, outputs and fp32 exact math
+ *  as bigru_infer_window, for a few windows at a time (B of 1 to ~16 is the intended use; any B works).  Per layer one
+ *  SGEMM forms the input projection of all T steps, then one thread-block cluster per (direction, group of up to 4
+ *  windows) walks the recurrence with its W_hh slices resident in shared memory, exchanging h through distributed shared
+ *  memory each step; a last kernel applies the pooling head, Linear and sigmoid.  2L+1 launches (2L+2 with d_xmin).
+ *  Hidden sizes above 256 need a 16-CTA (non-portable) cluster; where the device does not grant one, and for H > 512,
+ *  the call returns BIGRU_ERR_UNSUPPORTED with a message.  d_work: caller-owned device buffer, 16-byte aligned, of
+ *  bigru_infer_cluster_workspace_bytes() bytes for the same (B, T, F, H, L, bidirectional); the library never
+ *  allocates.  The workspace query needs no device. */
+int  bigru_infer_cluster_workspace_bytes(int B, int T, int F, int H, int L, int bidirectional, size_t* bytes);
+int  bigru_infer_cluster(const float* d_params, const float* d_x, const float* d_xmin, const float* d_xmax, int B, int T, int F,
+                         int H, int L, int C, int bidirectional, void* d_work, float* d_logits, float* d_probs, void* stream);
+/* The launch geometry bigru_infer_cluster picks on the current device for B windows of hidden size H: CTAs per cluster,
+ *  hidden units per CTA, windows per cluster, and cudaOccupancyMaxActiveClusters of that launch.  Needs the device. */
+int  bigru_infer_cluster_geometry(int B, int H, int bidirectional, int* cluster_ctas, int* units_per_cta, int* windows_per_cluster,
+                                  int* max_active_clusters);
+
 /* --- train_model/evaluate_model metrics (biGRU_model.py:213-221): pred = sigmoid(logit) > 0.5;
  *  d_counts[0] += #rows with all labels right; [1] += #label mismatches;
  *  [2+3c], [3+3c], [4+3c] += tp, fp, fn of class c.  int64 accumulators, caller zeroes. */
